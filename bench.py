@@ -10,11 +10,22 @@ prefill -> 512 decode steps.
   python bench.py --gpus N --steps K --warmup W            # this framework
   python bench.py --impl reference ...                      # CPU restatement of the
         reference path (oracle port; mlx itself is not installable offline)
+  python bench.py ... --dump-outputs DIR                    # + what the timed legs returned
 
 Prints ONE JSON line (rank 0).  `value` = decode tokens/s with inputs resident in
 HBM (CUDA events, max over ranks); `e2e` = the same request through the public
 API `generate(model, processor, prompt, image)` with a HOST image (preprocessing,
-pinned H2D of pixel_values, per-token D2H inside the timed region).
+pinned H2D of pixel_values, per-token D2H inside the timed region).  Every leg
+times exactly K steps (C5: K runs of the whole request set).
+
+--dump-outputs DIR (rank 0) writes, after each leg's timed steps, what its last
+timed step returned to its caller as DIR/<leg>_<name>.npy: float32 for floating
+point outputs (bf16 converts exactly), float64 for token ids.  Inputs and weights
+are seeded, so two builds run with the same arguments can be compared file by file.
+The GEMM configurations are picked by timing them at first use, and a different
+split of the K sum rounds differently (seen once in the C4 prefill on a B200 at
+1000 W: logits 3.5e-2 relative L2 apart between two runs of one build);
+B200_WT_TUNE=0 fixes them.
 """
 import argparse
 import json
@@ -31,6 +42,35 @@ sys.path.insert(0, ROOT)
 N_TEXT, N_OUT, IMG_HW = 128, 512, (336, 336)
 W_BYTES_2B = 3_087_428_608      # SURVEY §8(d): decode weight bytes / token (bf16, tied head)
 KV_BYTES_PER_POS = 28_672       # 2 (k,v) * 2 kv heads * 128 * 2 B * 28 layers
+DUMP_MAX_ELEMS = 1 << 20        # larger outputs are dumped as a fixed, seeded sample (all dumps stay < 64 MB)
+
+
+def dump_output(dump_dir, name, x):
+    """Write one output of a timed step as <dump_dir>/<name>.npy (--dump-outputs).
+    Floating point -> float32, integers (token ids) -> float64, both exact.  An output of more than
+    DUMP_MAX_ELEMS elements is flattened and sampled at positions fixed by its size and a constant seed."""
+    import numpy as np
+    import torch
+    if isinstance(x, torch.Tensor):
+        if x.is_cuda:
+            torch.cuda.synchronize(x.device)      # device outputs are written on the engine's stream
+        x = x.detach().cpu()
+        x = (x.float() if x.is_floating_point() else x).numpy()
+    x = np.asarray(x)
+    x = x.astype(np.float32 if np.issubdtype(x.dtype, np.floating) else np.float64)
+    if x.size > DUMP_MAX_ELEMS:
+        pick = np.random.default_rng(0).choice(x.size, DUMP_MAX_ELEMS, replace=False)
+        x = x.reshape(-1)[np.sort(pick)]
+    np.save(os.path.join(dump_dir, name + ".npy"), x)
+
+
+def _token_log(eng, n):
+    """the last `n` token ids the engine's greedy sampler wrote (prefill's first token + decode steps)"""
+    import torch
+    host = torch.empty(n, dtype=torch.int32).pin_memory()
+    eng.fetch_tokens(eng.tokens_launched - n, n, host)
+    eng.stream.synchronize()
+    return host
 
 
 # ViT + merge + LM prefill FLOPs of one C2 request (SURVEY §8d: 2*M*N*K per GEMM, 4*N^2*D attention)
@@ -235,20 +275,26 @@ def lockstep_2b(world, rank, dev, args, model, processor, ids, pvd, grid):
     def run():
         g = BatchGenerator(model, processor, max_tokens=n_out, completion_batch_size=rows, prefill_batch_size=rows,
                            decode_slice=32)
-        g.insert([prompt] * rows, [n_out] * rows, [dict(kw) for _ in range(rows)])
+        uids = g.insert([prompt] * rows, [n_out] * rows, [dict(kw) for _ in range(rows)])
+        toks = {u: [] for u in uids}
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
         t0 = time.perf_counter()
-        n = 0
         while g.has_work:
-            n += len(g.next()[1])
+            for r in g.next()[1]:
+                toks[r.uid].append(r.token)
         torch.cuda.synchronize()
-        return time.perf_counter() - t0, n
+        return time.perf_counter() - t0, [toks[u] for u in uids]
 
     run()
-    dt, n = run()
-    assert n == rows * n_out
+    dt = 0.0
+    for _ in range(args.steps):
+        t, toks = run()
+        dt += t / args.steps
+    assert all(len(t) == n_out for t in toks)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "c5_2b_rows_tokens", toks)
     step_ms = eng.last_decode_ms()
     t = torch.tensor([dt, step_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -257,7 +303,7 @@ def lockstep_2b(world, rank, dev, args, model, processor, ids, pvd, grid):
     peak, peak_src = _peaks()
     bytes_step = W_BYTES_2B + rows * KV_BYTES_PER_POS * (N_TEXT + 144 + n_out / 2)
     return {"workload": f"Qwen2-VL-2B, {rows} lock-step rows per GPU (the C2 request x {rows}), {n_out} tokens out each, "
-                        "admission + prefill of the rows inside the timed region",
+                        f"admission + prefill of the rows inside the timed region, seconds = mean of {args.steps} runs",
             "rows_per_gpu": rows, "seconds": dt, "tokens_per_s": world * rows * n_out / dt,
             "decode_ms_per_step": step_ms,
             "roofline": {"bound": "hbm", "achieved": bytes_step / (step_ms / 1e3) / 1e9 if step_ms > 0 else None,
@@ -320,8 +366,13 @@ def c5_leg(world, rank, dev, args):
         return time.perf_counter() - t0, toks
 
     run()                      # warm-up (GEMM configurations are measured on first use, graphs captured)
-    dt, toks = run()
+    dt = 0.0
+    for _ in range(args.steps):
+        t, toks = run()
+        dt += t / args.steps
     assert all(len(toks[i]) == n_out for i in shard_requests(n_req, world, rank))
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "c5_tokens", toks)      # every request's tokens (gathered over ranks)
     # device time of one lock-step step, from a dedicated slice of 64 steps on the warm engine
     step_ms = eng.last_decode_ms()
     t = torch.tensor([dt, step_ms], dtype=torch.float64, device=dev)
@@ -333,7 +384,8 @@ def c5_leg(world, rank, dev, args):
     bytes_step = W_BYTES_7B + rows * KV_BYTES_PER_POS_7B * mean_ctx
     out = {"workload": f"C5: Qwen2-VL-7B bf16, {n_req} concurrent requests ({rows} per GPU) over {world} GPU(s), "
                        f"1x336x336 image + 128 text tokens in, {n_out} out each, continuous batching "
-                       "(lock-step rows, one weight stream per step), router: request i -> rank i mod N",
+                       "(lock-step rows, one weight stream per step), router: request i -> rank i mod N, "
+                       f"seconds = mean of {args.steps} runs",
            "requests": n_req, "rows_per_gpu": rows, "seconds": dt,
            "requests_per_s": n_req / dt, "tokens_per_s": n_req * n_out / dt,
            "tokens_per_s_per_gpu": rows * n_out / dt,
@@ -382,31 +434,39 @@ def c3_leg(dev, args):
         ev[1].record(eng.stream)
         embs = [model.get_input_embeddings(ids, pv, cached_image_features=feats[b:b + 1]).inputs_embeds for b in range(B)]
         if args.c3_sequential:      # A/B: one prefill call per request
-            for b in range(B):
-                lm(ids, inputs_embeds=embs[b], cache=make_prompt_cache(lm), logits_to_keep=1, reserve_tokens=T + 8)
+            out = [lm(ids, inputs_embeds=embs[b], cache=make_prompt_cache(lm), logits_to_keep=1,
+                      reserve_tokens=T + 8).logits for b in range(B)]
         else:                       # the 8 prompts in ONE pass over the weights (reference PromptProcessingBatch)
             rows, _ = lm.make_batch_cache(B, T + 8)
-            lm.prefill_rows([ids] * B, embs, [lm.make_cache_row(rows.pool, b) for b in range(B)], reserve_tokens=T + 8)
+            out = lm.prefill_rows([ids] * B, embs, [lm.make_cache_row(rows.pool, b) for b in range(B)],
+                                  reserve_tokens=T + 8)
         ev[2].record(eng.stream)
         eng.stream.synchronize()
-        return ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2])
+        return ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), feats, out
 
     for _ in range(3):
         step()
-    K = max(2, min(args.steps, 5))
+    K = args.steps
     torch.cuda.synchronize()
     sampler = ClockSampler(dev.index or 0)     # this leg is the power-hungry one (dense tcgen05 work for ~0.1 s per step)
     sampler.start()
     t0 = time.perf_counter()
     tw, pf, per_step = 0.0, 0.0, []
     for _ in range(K):
-        a, b = step()
+        feats = out = None              # the previous step's outputs are freed before the next step allocates
+        a, b, feats, out = step()
         tw += a
         pf += b
         per_step.append(round(b, 2))
     torch.cuda.synchronize()
     wall = (time.perf_counter() - t0) / K
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "c3_image_features", feats)
+        if args.c3_sequential:
+            dump_output(args.dump_outputs, "c3_prefill_logits", torch.cat(out))
+        else:
+            dump_output(args.dump_outputs, "c3_first_tokens", out)
     tw, pf = tw / K, pf / K
     E, I, nh = v.hidden_size, v.intermediate_size, v.num_attention_heads
     L = P + 1
@@ -471,22 +531,28 @@ def c4_leg(dev, args):
         ev[1].record(eng.stream)
         emb = model.get_input_embeddings(ids, pv_host, cached_image_features=feats)
         cache = make_prompt_cache(lm)
-        lm(ids, inputs_embeds=emb.inputs_embeds, cache=cache, logits_to_keep=1, reserve_tokens=T + n_out + 1)
+        out = lm(ids, inputs_embeds=emb.inputs_embeds, cache=cache, logits_to_keep=1, reserve_tokens=T + n_out + 1)
         ev[2].record(eng.stream)
         lm.fused_greedy_decode_n(n_out, cache, reserve_tokens=T + n_out + 1)
         ev[3].record(eng.stream)
         eng.stream.synchronize()
-        return ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3])
+        return (ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3])), feats, out.logits
 
     for _ in range(2):
         step()
-    K = max(2, min(args.steps, 3))
+    K = args.steps
     l0 = eng.launch_count
     acc = [0.0, 0.0, 0.0]
     for _ in range(K):
-        for i, x in enumerate(step()):
+        feats = logits = None           # the previous step's outputs are freed before the next step allocates
+        times, feats, logits = step()
+        for i, x in enumerate(times):
             acc[i] += x / K
     launches = (eng.launch_count - l0) / K
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "c4_image_features", feats)
+        dump_output(args.dump_outputs, "c4_prefill_logits", logits)
+        dump_output(args.dump_outputs, "c4_tokens", _token_log(eng, n_out + 1))
     tw, pf, dec = acc
     H, Il = t.hidden_size, t.intermediate_size
     hd = H // t.num_attention_heads
@@ -529,9 +595,19 @@ def main():
     ap.add_argument("--no-mega", action="store_true")
     ap.add_argument("--mega-mode", type=int, default=None,
                     help="decode kernel: 0 per-phase kernels, 1 k_mega (CUDA cores), 2 k_mega_tc (tcgen05)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each leg's last timed step returned as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the outputs of the b200 implementation")
 
     rank = int(os.environ.get("RANK", "0"))
+    if rank != 0:
+        args.dump_outputs = None          # rank 0 writes the outputs (C5 tokens are gathered from every rank)
+    elif args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     import numpy as np
@@ -624,18 +700,18 @@ def main():
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
 
     def device_step():
-        """one request with inputs resident in HBM; returns (prefill_ms, decode_ms)."""
+        """one request with inputs resident in HBM; returns (prefill_ms, decode_ms, embeddings, prefill logits)."""
         cache = make_prompt_cache(model.language_model)
         ev[0].record(eng.stream)
         emb = model.get_input_embeddings(ids, pvd, image_grid_thw=grid)
-        model.language_model(ids, inputs_embeds=emb.inputs_embeds, cache=cache,
-                             position_ids=emb.position_ids, rope_deltas=emb.rope_deltas,
-                             logits_to_keep=1, reserve_tokens=T + N_OUT + 1)
+        out = model.language_model(ids, inputs_embeds=emb.inputs_embeds, cache=cache,
+                                   position_ids=emb.position_ids, rope_deltas=emb.rope_deltas,
+                                   logits_to_keep=1, reserve_tokens=T + N_OUT + 1)
         ev[1].record(eng.stream)
         model.language_model.fused_greedy_decode_n(N_OUT, cache, reserve_tokens=T + N_OUT + 1)
         ev[2].record(eng.stream)
         eng.stream.synchronize()
-        return ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2])
+        return ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), emb.inputs_embeds, out.logits
 
     def barrier():
         torch.cuda.synchronize()
@@ -652,13 +728,19 @@ def main():
     t0 = time.perf_counter()
     pre_ms, dec_ms = 0.0, 0.0
     for _ in range(args.steps):
-        a, b = device_step()
+        embeds = logits = None          # the previous step's outputs are freed before the next step allocates
+        a, b, embeds, logits = device_step()
         pre_ms += a
         dec_ms += b
     barrier()
     wall = time.perf_counter() - t0
     launches = eng.launch_count - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "c2_inputs_embeds", embeds)
+        dump_output(args.dump_outputs, "c2_prefill_logits", logits)
+        dump_output(args.dump_outputs, "c2_tokens", _token_log(eng, N_OUT + 1))
+        dump_output(args.dump_outputs, "c2_last_logprobs", eng.snapshot("logprobs"))
 
     # ---- e2e through the public API with a host image --------------------------
     def e2e_step():
@@ -678,6 +760,8 @@ def main():
         e2e_prompt_tps.append(r.prompt_tps)
         assert r.generation_tokens == N_OUT
     barrier()
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "e2e_last_logprobs", r.logprobs)
 
     c5 = None
     if not args.no_c5:

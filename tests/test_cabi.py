@@ -67,10 +67,8 @@ def test_no_oracle_import_in_product():
 
 
 def test_engine_refuses_without_gpu():
+    """a model placed on the CPU gets no engine, whether or not the machine has a GPU"""
     import pytest
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
     from mlx_vlm_b200 import _native as N
     from mlx_vlm_b200.models.qwen2_vl import Model
     from mlx_vlm_b200.models.qwen2_vl.config import qwen2_vl_2b_config
